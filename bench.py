@@ -2,6 +2,7 @@
 """Benchmark of the offline Paraformer hot path (BASELINE.json metric: RTFx = audio-seconds / second).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--mode fp32|fp16x3|fp16x6|fp16] [--impl reference]
+                  [--dump-outputs DIR]
 
 One step = one pass of the hot path over one job of synthetic 16 kHz utterances (BASELINE.json `configs`):
   --config 2 (default, the configuration the metric is quoted on): Paraformer-large, 64 x 30 s per GPU, weak scaling
@@ -572,6 +573,19 @@ def parity_block(job, parity_path, last_ids):
     return out
 
 
+def dump_outputs(out_dir, ids):
+    """--dump-outputs: what a caller of the timed path receives from its last step, the greedy token ids of every utterance of the
+    job in input order, so that two builds can be compared output for output on the same seeded inputs.  float64 (ids are exact):
+    token_ids.npy [utterances, longest] padded with -1, token_lens.npy [utterances]; under 1 MB for every config."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = [[int(t) for t in r] for r in ids]
+    out = np.full((len(rows), max((len(r) for r in rows), default=0)), -1.0, dtype=np.float64)
+    for i, r in enumerate(rows):
+        out[i, :len(r)] = r
+    np.save(os.path.join(out_dir, "token_ids.npy"), out)
+    np.save(os.path.join(out_dir, "token_lens.npy"), np.array([len(r) for r in rows], dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -585,7 +599,11 @@ def main():
     ap.add_argument("--parity-out", default=None, help="(reference leg) write the oracle's ids / log-probs of the sample here")
     ap.add_argument("--port", action="store_true", help="(reference leg) time the oracle port even when the reference imports")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the token ids of the last timed step to DIR/token_ids.npy and DIR/token_lens.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the timed GPU path's outputs; --impl reference times a CPU sample of the job instead")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -641,6 +659,8 @@ def main():
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms.item())
     last_ids = job.runner_dev.finish(h, job.plan["n_total"])       # id lists of the last timed job, all utterances, input order
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_ids)
     toks = torch.cat([t.float() for t in job.tok_stats]) if job.tok_stats else torch.zeros(1)
     ntok_mean, n_max = float(toks.mean()), int(toks.max())
     log("device-resident: %.2f ms/step" % (ms_total / args.steps))

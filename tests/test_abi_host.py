@@ -13,6 +13,7 @@ import torch
 from conftest import GOLDEN, ROOT
 
 import funasr_b200
+import ref_shim
 from funasr_b200 import _abi, synth
 from funasr_b200.engine import kaldi_mel_banks, num_lfr_frames
 from funasr_b200.sharding import shard_utterances
@@ -169,12 +170,11 @@ def test_gather_token_ids_two_ranks_gloo(tmp_path):
     assert all("ok" in o for o in outs)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/funasr"), reason="live reference not present")
+@pytest.mark.skipif(not ref_shim.reference_available(), reason="needs the FunASR package itself (the unmodified reference)")
 def test_plugs_into_reference_tables_and_automodel_build():
     """Drop-in surface against the real FunASR: classes land in funasr.register.tables and AutoModel.build_model
     constructs ParaformerB200 + WavFrontendB200 and strict-loads a checkpoint via load_pretrained_model (CPU build
     only — running it needs a GPU)."""
-    import ref_shim
     ref_shim.import_reference()
     from funasr.register import tables
     funasr_b200.install()
@@ -288,22 +288,33 @@ def test_header_is_plain_c_and_links(tmp_path):
 
 def test_funoffline_client_links_against_the_reference_header(tmp_path):
     """Link compatibility of the C++ runtime surface: the client of examples/offline_runtime_client.cpp (the call sequence of
-    runtime/onnxruntime/bin/funasr-onnx-offline.cpp) compiled against the REFERENCE's own funasrruntime.h (when /root/reference is
-    present; this repo's copy of the declarations otherwise) links against libfunasr_b200.so — same names, same C++ argument types,
-    so the mangled symbols resolve — and fails cleanly (no CPU path, no model) when run without a GPU."""
+    runtime/onnxruntime/bin/funasr-onnx-offline.cpp) compiled against the REFERENCE's own funasrruntime.h needs the mangled entry
+    points stored in tests/golden/funasrruntime_client_symbols.txt (oracle/make_runtime_symbols_golden.py): libfunasr_b200.so
+    defines every one of them — same names, same C++ argument types — and this repo's copy of the declarations asks for exactly
+    that set.  The client built against this repo's header (and, when the reference tree is present, against its header too)
+    links and fails cleanly (no CPU path, no model) when run without a GPU."""
     import shutil
+    import make_runtime_symbols_golden as mk
     if shutil.which("g++") is None:
         pytest.skip("no g++")
-    ref_hdr = "/root/reference/runtime/onnxruntime/include/funasrruntime.h"
+    with open(os.path.join(GOLDEN, "funasrruntime_client_symbols.txt")) as f:
+        want = f.read().split()
+    assert len(want) == 15
+    lib = ctypes.CDLL(_abi.LIB_PATH)
+    assert [s for s in want if not hasattr(lib, s)] == []
+    assert mk.client_runtime_symbols('"funasrruntime_b200.h"', os.path.join(ROOT, "include")) == want
     exe = str(tmp_path / "client")
-    for hdr, inc in ((('"funasrruntime.h"', os.path.dirname(ref_hdr)),) if os.path.exists(ref_hdr) else ()) + (('"funasrruntime_b200.h"', os.path.join(ROOT, "include")),):
+    headers = [('"funasrruntime_b200.h"', os.path.join(ROOT, "include"))]
+    if os.path.exists(os.path.join(mk.reference_header_dir(), "funasrruntime.h")):
+        headers.append(('"funasrruntime.h"', mk.reference_header_dir()))
+    for hdr, inc in headers:
         cmd = ["g++", "-std=c++17", "-DFUNASR_RUNTIME_HEADER=" + hdr, "-I" + inc, "-I" + os.path.join(ROOT, "include"),
                os.path.join(ROOT, "examples", "offline_runtime_client.cpp"), "-L" + os.path.join(ROOT, "funasr_b200"), "-lfunasr_b200",
                "-Wl,-rpath," + os.path.join(ROOT, "funasr_b200"), "-o", exe]
         r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
         assert r.returncode == 0, r.stdout[-2000:]
-    r = subprocess.run([exe, str(tmp_path), str(tmp_path / "none.wav")], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
-    assert r.returncode == 1 and "init failed" in r.stdout
+        r = subprocess.run([exe, str(tmp_path), str(tmp_path / "none.wav")], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+        assert r.returncode == 1 and "init failed" in r.stdout
 
 
 def test_product_never_touches_the_oracle_or_the_reference_tree():

@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import (BICIF_CASES, CTX_CASES, GOLDEN_CASES, SEACO_CASES, SV_CASES, gold_stamps, load_bicif_case, load_case, load_ctx_case,
+from conftest import (BICIF_CASES, CTX_CASES, GOLDEN, GOLDEN_CASES, SEACO_CASES, SV_CASES, gold_stamps, load_bicif_case, load_case, load_ctx_case,
                       load_seaco_case, load_sv_case,
                       rel_err, state_dict_for)
 
@@ -87,35 +87,25 @@ def test_lfr_equals_reference_formula():
         assert torch.equal(ref_lfr(x, 7, 6), O.apply_lfr(x, 7, 6)), T
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="live reference tree not present")
 def test_oracle_matches_live_reference_components():
-    """Run the reference's own classes (from /root/reference) on fresh random inputs and compare stage by stage."""
-    ref_shim.import_reference()
-    from funasr.register import tables
+    """The reference's own SANMEncoder and CifPredictorV2 on seeded random inputs, compared stage by stage: their outputs as stored
+    in tests/golden/live_components.npz (oracle/make_live_golden.py) and, when the reference is importable, a fresh run of them."""
+    import make_live_golden as mk
     from funasr_b200 import synth
     cfg = synth.PARAFORMER_TINY
-    p = synth.make_state_dict(cfg, 11)
-    enc = tables.encoder_classes["SANMEncoder"](input_size=560, output_size=512, attention_heads=4, linear_units=2048,
-                                                num_blocks=cfg.enc_layers, input_layer="pe", kernel_size=11, sanm_shfit=0,
-                                                selfattention_layer_type="sanm").eval()
-    enc.load_state_dict({k[len("encoder."):]: v for k, v in p.items() if k.startswith("encoder.")}, strict=True)
-    pred = tables.predictor_classes["CifPredictorV2"](idim=512, threshold=1.0, l_order=1, r_order=1, tail_threshold=0.45).eval()
-    pred.load_state_dict({k[len("predictor."):]: v for k, v in p.items() if k.startswith("predictor.")}, strict=True)
-    g = torch.Generator().manual_seed(5)
-    feats = torch.randn(3, 41, 560, generator=g)
-    lens = torch.tensor([41, 17, 30], dtype=torch.int32)
-    for b in range(3):
-        feats[b, lens[b]:] = 0
+    p, feats, lens = mk.component_inputs()
+    runs = [{k: torch.from_numpy(v) for k, v in mk.load_components(os.path.join(GOLDEN, "live_components.npz")).items()}]
+    if ref_shim.reference_available():
+        ref_shim.import_reference()
+        runs.append({k: torch.from_numpy(v) for k, v in mk.run_components().items()})
     with torch.no_grad():
-        r_enc, r_len, _ = enc(feats, lens)
         o_enc, o_len = O.encoder(feats, lens, p, cfg.enc_layers)
-        assert torch.allclose(r_enc, o_enc, rtol=0, atol=1e-5) and r_len.tolist() == o_len.tolist()
-        mask = (torch.arange(41)[None, :] < lens[:, None])[:, None, :]
-        r_emb, r_tok, r_al, r_pk = pred(r_enc, None, mask, ignore_id=-1)
-        o_emb, o_tok, o_al, o_pk = O.predictor(r_enc, lens, p)
-        assert r_tok.tolist() == o_tok.tolist()
-        assert torch.allclose(r_al, o_al, atol=1e-6) and torch.allclose(r_pk, o_pk, atol=1e-5)
-        assert torch.allclose(r_emb, o_emb, atol=1e-4)
+        for r in runs:
+            assert torch.allclose(r["enc"], o_enc, rtol=0, atol=1e-5) and r["enc_lens"].tolist() == o_len.tolist()
+            o_emb, o_tok, o_al, o_pk = O.predictor(r["enc"], lens, p)
+            assert r["token_num"].tolist() == o_tok.tolist()
+            assert torch.allclose(r["alphas"], o_al, atol=1e-6) and torch.allclose(r["peaks"], o_pk, atol=1e-5)
+            assert torch.allclose(r["acoustic"], o_emb, atol=1e-4)
 
 
 @pytest.mark.parametrize("name", list(SV_CASES))

@@ -1,10 +1,13 @@
 """Property tests (hypothesis) of the host-side logic around the hot path: utterance sharding, length bucketing, frame
 arithmetic and the CIF timestamp routine.  CPU only."""
+import json
 import os
 
 import numpy as np
 import pytest
 from hypothesis import given, settings, strategies as st
+
+from conftest import GOLDEN
 
 from funasr_b200.batching import bucket_by_length, padding_efficiency, run_bucketed
 from funasr_b200.engine import num_lfr_frames
@@ -67,8 +70,8 @@ def test_timestamps_are_ordered_and_inside_the_utterance(alphas, n_tok, rate, of
 
 
 def test_hotword_list_follows_reference_seg_dict_rules(tmp_path):
-    """funasr_b200.hotwords.generate_hotwords_list against the reference's own function (contextual_paraformer/model.py:528-660)
-    when /root/reference is importable, and against hand-derived expectations otherwise: seg_dict lookup (lower-cased), per-character
+    """funasr_b200.hotwords.generate_hotwords_list against hand-derived expectations and the stored outputs of the reference's own
+    function (contextual_paraformer/model.py:528-660): seg_dict lookup (lower-cased), per-character
     fallback for CJK / digit words, <unk> for the rest, [sos] terminator; .txt files and plain strings."""
     from funasr_b200.hotwords import generate_hotwords_list, seg_tokenize
 
@@ -98,18 +101,14 @@ def test_hotword_list_follows_reference_seg_dict_rules(tmp_path):
     assert generate_hotwords_list("gpu Hello", Tok(), Fe(), sos=1) == [[8], [9], [1]]
     with pytest.raises(ValueError):
         generate_hotwords_list("http://example.com/hw.txt", Tok(), fe, sos=1)
-    if os.path.isdir("/root/reference"):
-        import sys
-        sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-        import ref_shim
-        ref_shim.import_reference()
-        from funasr.models.contextual_paraformer.model import ContextualParaformer
-
-        class Dummy:
-            sos = 1
-        for src in ["Hello 你好 GPU xyz", str(txt)]:
-            want = ContextualParaformer.generate_hotwords_list(Dummy(), src, tokenizer=Tok(), frontend=fe)
-            assert generate_hotwords_list(src, Tok(), fe, sos=1) == want
+    # the reference's own function on the same string and file (tests/golden/live_host.json, oracle/make_live_golden.py)
+    import make_live_golden as mk
+    assert Tok.vocab == mk.HotwordTokenizer.vocab
+    assert ((tmp_path / "seg_dict").read_text(encoding="utf8"), txt.read_text(encoding="utf8")) == (mk.HOTWORD_SEG_DICT, mk.HOTWORD_FILE)
+    with open(os.path.join(GOLDEN, "live_host.json"), encoding="utf8") as f:
+        want = json.load(f)["hotwords"]
+    assert generate_hotwords_list(mk.HOTWORD_STRING, Tok(), fe, sos=1) == want["string"]
+    assert generate_hotwords_list(str(txt), Tok(), fe, sos=1) == want["file"]
 
 
 def test_bench_flop_model_matches_the_survey_figures():
@@ -154,3 +153,15 @@ def test_bench_stage_tap_comparison():
     del dump["tap_feats"], dump["tap_alphas"]
     assert set(bench.compare_taps(dump, dict(full, acoustic=got["acoustic"]))) == {"enc", "acoustic"}
     assert "error" in bench.compare_taps(dump, dict(full, enc=full["enc"][:, :40], acoustic=got["acoustic"]))["enc"]
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: every utterance's ids in input order, padded with -1, lengths beside them, float64 (ids exact)."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod3", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    bench.dump_outputs(str(tmp_path / "out"), [[5, 8404, 3], [], [7]])
+    ids, lens = np.load(tmp_path / "out" / "token_ids.npy"), np.load(tmp_path / "out" / "token_lens.npy")
+    assert ids.dtype == np.float64 and lens.dtype == np.float64
+    assert ids.tolist() == [[5, 8404, 3], [-1, -1, -1], [7, -1, -1]] and lens.tolist() == [3, 0, 1]

@@ -41,25 +41,20 @@ def test_cif_wo_hidden_is_the_running_integral():
 
 
 def test_timestamps_against_live_reference_if_available():
-    try:
-        from oracle import ref_shim
+    """The Paraformer call of the reference's ts_prediction_lfr6_standard on 50 seeded cases: its outputs as stored in
+    tests/golden/live_host.json (oracle/make_live_golden.py) and, when the reference is importable, a fresh run of it."""
+    import make_live_golden as mk
+    import ref_shim
+    with open(os.path.join(GOLDEN, "live_host.json"), encoding="utf8") as f:
+        runs = [json.load(f)["timestamps"]]
+    if ref_shim.reference_available():
         ref_shim.import_reference()
-        import torch
-        from funasr.utils.timestamp_tools import ts_prediction_lfr6_standard as ref_fn
-    except Exception:
-        pytest.skip("reference not importable here (GPU box)")
-    rng = np.random.default_rng(7)
-    for trial in range(50):
-        T = int(rng.integers(6, 120))
-        a = (rng.random(T).astype(np.float32) ** 2 * 0.8).astype(np.float32)
-        peaks = TS.cif_wo_hidden(a, 1.0)
-        chars = ["c%d" % i for i in range(max(1, int((peaks >= 1 - 1e-4).sum()) - 1 + trial % 2))]
-        try:
-            want = ref_fn(torch.tensor(peaks.copy()), torch.tensor(a.copy()), copy.copy(chars), upsample_rate=1)
-        except IndexError:
-            want = ("", [])
-        got = TS.paraformer_timestamps(peaks, a, chars)
-        assert got[1] == want[1] and got[0] == want[0]
+        runs.append(mk.run_timestamps())
+    for want in runs:
+        assert len(want) == 50
+        for (a, peaks, chars), (w_txt, w_stamps) in zip(mk.timestamp_inputs(), want):
+            got = TS.paraformer_timestamps(peaks, a, copy.copy(chars))
+            assert got[1] == w_stamps and got[0] == w_txt
 
 
 def test_stamps_only_path_equals_the_labelled_walk():

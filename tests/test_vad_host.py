@@ -1,6 +1,7 @@
 """CPU: the FSMN-VAD host logic (funasr_b200/vad.py: end-point detector, the reference's chunked frame delivery, the dynamic
 end-silence schedule) and the oracle restatement of the VAD scores (oracle/vad_oracle.py) against golden vectors produced by the
 UNMODIFIED reference (oracle/make_vad_golden.py: FsmnVADStreaming + WavFrontendOnline through AutoModel.generate)."""
+import json
 import os
 
 import numpy as np
@@ -69,14 +70,17 @@ def test_merge_vad_matches_reference_function():
     segs = [[0, 2450], [2990, 7940], [8970, 11440], [11990, 16920], [17970, 20440], [21030, 25940], [27000, 40000]]
     assert vad.merge_vad(segs, 15000) == [[0, 11990], [11990, 25940], [25940, 40000]]
     assert vad.merge_vad([[5, 9]], 15000) == [[5, 9]]
-    if os.path.isdir("/root/reference/funasr"):
-        import ref_shim
-        ref_shim.import_reference()
-        from funasr.utils.vad_utils import merge_vad as ref_merge
-        g = np.random.default_rng(0)
-        for _ in range(50):
-            t = np.sort(g.integers(0, 200000, size=2 * int(g.integers(1, 12)))).reshape(-1, 2).tolist()
-            assert vad.merge_vad([list(x) for x in t], 15000) == ref_merge([list(x) for x in t], 15000)
+    # the reference's funasr.utils.vad_utils.merge_vad on 50 seeded segment lists (tests/golden/live_host.json, oracle/make_live_golden.py)
+    import make_live_golden as mk
+    want = _live_host()["merge_vad"]
+    assert len(want) == 50
+    for t, w in zip(mk.merge_vad_inputs(), want):
+        assert vad.merge_vad([list(x) for x in t], 15000) == w
+
+
+def _live_host():
+    with open(os.path.join(GOLDEN, "live_host.json"), encoding="utf8") as f:
+        return json.load(f)
 
 
 def _flat_decibels(n_samples):
@@ -89,29 +93,32 @@ def test_detector_matches_the_reference_runtimes_compiled_cpp_detector():
     """Second, independent pin of the end-point state machine: the reference's C++ runtime carries its own implementation
     (runtime/onnxruntime/src/e2e-vad.h, header-only; compiled from the reference tree by oracle/knf/Makefile and called like
     fsmn-vad.cpp:245-249).  It has no dynamic end-silence schedule, so funasr_b200/vad.py is run with a fixed max_end_silence_time.
-    Checked against the committed outputs of that detector (tests/golden/vad_cpp_detector.npz, oracle/make_vad_cpp_golden.py) and —
-    when the compiled library is present — live on fresh random posteriors (incl. recordings beyond the 60 s chunk / segment limit)
-    and on the Python reference's own scores of the fixed-schedule golden cases."""
+    Checked against the committed outputs of that detector (tests/golden/vad_cpp_detector.npz, oracle/make_vad_cpp_golden.py), on
+    seeded random posteriors (incl. recordings beyond the 60 s chunk / segment limit) against its stored segments
+    (tests/golden/live_host.json, oracle/make_live_golden.py) and — when the compiled library is present — against a live run, and on the
+    Python reference's own scores of the fixed-schedule golden cases."""
     import knf_ref
-    import make_vad_cpp_golden as mk
+    import make_live_golden as mk
     g = np.load(os.path.join(GOLDEN, "vad_cpp_detector.npz"))
     for i, (n, mes, thr10) in enumerate(g["meta"].tolist()):
         sp = (g["sil_prob_%d" % i].astype(np.float32) / 1024).tolist()
         got = vad.detect_segments(sp, _flat_decibels(n), n, max_end_silence_time=mes, speech_noise_thres=thr10 / 10)
         assert got == g["segments_%d" % i].tolist(), i
-    if not knf_ref.build():
-        return                                          # no reference tree and no prebuilt library: the fixture above is the check
-    rng = np.random.default_rng(7)
-    for it in range(60):
-        n, sp, wav, mes, thr = mk.random_case(rng, 40.0 if it < 50 else 150.0)
-        want = knf_ref.vad_segments(sp, wav, mes, 60000, thr)
+    stored = _live_host()["vad_cpp"]
+    have = knf_ref.build()
+    for it, (n, sp, wav, mes, thr) in enumerate(mk.vad_cpp_random_inputs()):
+        want = stored["random"][it]
+        if have:
+            assert knf_ref.vad_segments(sp, wav, mes, 60000, thr) == want, it
         db = VO.frame_decibels(torch.from_numpy(wav)).double().tolist()
         assert vad.detect_segments(sp.tolist(), db, n, max_end_silence_time=mes, speech_noise_thres=thr) == want, it
-    for name in ("vad_fixed800", "vad_short", "vad_silence"):        # the Python reference's scores through the C++ detector
+    for name in mk.VAD_GOLDEN_CASES:                                 # the Python reference's scores through the C++ detector
         seconds, seed, pattern, _ = VAD_CASES[name]
         gg = _gold(name)
-        wav = synth.make_vad_wav(seconds, seed, pattern).numpy()
-        assert knf_ref.vad_segments(gg["sil_prob"], wav, 800, 60000, 0.6) == gg["segments"].tolist()
+        assert stored["golden_scores"][name] == gg["segments"].tolist()
+        if have:
+            wav = synth.make_vad_wav(seconds, seed, pattern).numpy()
+            assert knf_ref.vad_segments(gg["sil_prob"], wav, 800, 60000, 0.6) == gg["segments"].tolist()
 
 
 @pytest.mark.parametrize("name", list(VAD_CASES))
